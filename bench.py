@@ -11,6 +11,8 @@ reference's EM loop) and the equivalent EM iterations/s; HBM GB/s against the ro
   python bench.py --workload C4                          # Gibbs sampler (BASELINE configs[3]): chain-sweeps/s
   python bench.py --workload MODEL                       # one model round (K1 + K2 with posteriors + K3), rounds 1-10
   python bench.py --impl reference                       # oracle/_ref/rsem-run-em (the unmodified reference) on the host cores
+  python bench.py --dump-outputs DIR                     # also write what the last timed step returned to DIR/*.npy
+                                                         # (float64), to compare two builds (EM workloads and C4)
 
 A "step" is one EM round = K2 (E-step + count accumulation) [+ NCCL allreduce of the count vector when N > 1] + K4 (theta
 update, convergence test) over the resident hit matrix.  The matrix (>= 9 GB at C3) is far larger than L2 (126 MB), so
@@ -411,6 +413,9 @@ def run_ours(args):
     barrier()
     launches = ctx.launch_count() - l0
     cta_ns = ctx.estep_cta_times().astype(np.float64)
+    if args.dump_outputs and rank == 0:
+        # what em_rounds hands its caller after the last timed step: theta and that round's (sum, bchange, totnum)
+        dump_outputs(args.dump_outputs, theta=ctx.get_theta(), round_stats=np.array(stats[-1], np.float64))
     # keep the same load running until nvidia-smi has a few samples of it (a 20-round region lasts 50 ms)
     extra = 0
     while world == 1 and sampler.count_since(t_load0) < 5 and time.time() - t_load0 < 2.5:
@@ -554,6 +559,14 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(d, **arrays):
+    """writes each array as DIR/<name>.npy in float64; the inputs of every workload are seeded, so two builds run with the
+    same arguments can be compared file by file"""
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, f"{name}.npy"), np.ascontiguousarray(a, np.float64))
+
+
 def sort_rows_torch(torch, row_ptr, sid, conprb, ncpv, by):
     """Experiment: rows reordered by their first transcript id or by their degree."""
     N = row_ptr.numel() - 1
@@ -676,7 +689,8 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 20; MODEL times the model rounds 3-10 of rsem-run-em, so 8 there)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C3", choices=sorted(WORKLOADS) + ["C4", "MODEL"])
@@ -696,7 +710,23 @@ def main():
     ap.add_argument("--gibbs-reads", type=int, default=10_000_000)
     ap.add_argument("--gibbs-chains", type=int, default=8)
     ap.add_argument("--model-reads", type=int, default=2_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned as DIR/<name>.npy: theta and the round statistics (EM "
+                         "workloads), the last count vector of every chain and the posterior sums (C4)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "MODEL"):
+        # MODEL times whole rsem-run-em processes: their outputs are files in a temporary directory, and the drop-in
+        # tests compare those files with the reference's
+        ap.error("--dump-outputs covers --impl ours with the EM workloads (C1, C2, C3, C5) and C4")
+    if args.impl == "ours" and args.workload == "MODEL":
+        # only rounds 1-10 of rsem-run-em update the model; rounds 1-2 carry the first launches, so 3-10 are timed
+        if args.steps not in (None, 8):
+            ap.error("--workload MODEL times the 8 model rounds 3-10 of rsem-run-em: --steps must be 8")
+        args.steps = 8
+    elif args.steps is None:
+        args.steps = 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     # pin the OpenMP threads of the cpu_baseline leg before any OpenMP runtime starts
     os.environ.setdefault("OMP_PROC_BIND", "spread")

@@ -111,15 +111,22 @@ def run_gibbs(args):
         dt = time.perf_counter() - t0
         print(f"bench C4: gibbs_run burn-in {burnin}, {per_chain} samples per chain x {chains} chains: {dt:.2f} s", file=sys.stderr, flush=True)
         assert np.all(cv.sum(axis=1) == N + int(n0))  # every read is assigned to exactly one entry in every kept sample
-        return dt
+        return dt, cv, sums
 
     run(2, 1)  # warm-up (allocations, first launch)
     W = max(args.warmup, 3)
     K = args.steps
     # W + 1 sweeps per chain, then W + 1 + K: the difference times exactly K sweeps (x chains) through the whole C-ABI call;
     # each twice, the faster one counts (allocation / first-touch noise of a call is of the order of 0.1 s)
-    t_short = min(run(W, 1), run(W, 1))
-    t_long = min(run(W, 1 + K), run(W, 1 + K))
+    t_short = min(run(W, 1)[0], run(W, 1)[0])
+    t_long1 = run(W, 1 + K)[0]
+    t_long2, cv, sums = run(W, 1 + K)
+    t_long = min(t_long1, t_long2)
+    if args.dump_outputs:
+        # all kept count vectors would be chains x (1 + K) x (M + 1) values: the last one of every chain is written
+        last = cv.reshape(chains, 1 + K, M + 1)[:, -1, :]
+        bench.dump_outputs(args.dump_outputs, last_count_vectors=last, sum_c=sums[0], sum_c2=sums[1], sum_tpm=sums[2],
+                           sum_fpkm=sums[3], sum_gene_c2=sums[4])
     per_sweep_all = (t_long - t_short) / K          # one sweep of all chains, seconds
     chain_sweeps_per_s = chains / per_sweep_all
     # SURVEY.md 8(d): bytes per chain-sweep when C chains share the stream = (12 E + 8 N) / C + 8 N
@@ -199,14 +206,14 @@ def run_model(args):
     if rc != 0:
         print(json.dumps({"metric": "model_round_hits_per_sec", "error": err[-400:]}))
         return
-    per_round = (stamps[10] - stamps[2]) / 8   # rounds 3..10 (round 1-2 carry the first launches)
+    per_round = (stamps[2 + args.steps] - stamps[2]) / args.steps   # rounds 3..10 (rounds 1-2 carry the first launches)
     phases = [l for l in err.splitlines() if "phase timing" in l]
     # SURVEY 8(d) "K1/K3 rounds": per read its bases + qualities once per kernel, per hit 2 L reference bases + hit fields
     k1 = N * 4 * L + H * (2 * L + 4 + 4 + 4 + 8)
     k3 = N * 4 * L + H * (2 * L + 4 + 4 + 4 + 8)
     k2 = 12 * H + 16 * N + 8 * H + 8 * N
     peak, peak_src = bench.measured_peak_gbs()
-    out = {"metric": "model_round_hits_per_sec", "value": H / per_round, "unit": "hits/s", "n_gpus": 1, "steps": 8, "warmup": 2,
+    out = {"metric": "model_round_hits_per_sec", "value": H / per_round, "unit": "hits/s", "n_gpus": 1, "steps": args.steps, "warmup": 2,
            "ms_per_step": per_round * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
            "dtype": "f64", "data": "synthetic",
            "config": {"workload": f"MODEL: one model-updating EM round (K1 conprb + K2 with posteriors + K3 statistics + host "

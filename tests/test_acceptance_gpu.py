@@ -62,8 +62,11 @@ def _compare_tables(a, b):
 
 @pytest.fixture(scope="module")
 def installs(tmp_path_factory, built):
-    if not (rf.have_ref() and os.path.exists(DRIVER) and shutil.which("perl")):
-        pytest.skip("needs oracle/_ref with the Perl driver (oracle/Makefile) and perl")
+    if not (rf.have_ref() and os.path.exists(DRIVER)):
+        pytest.skip("oracle/_ref with the reference's Perl driver is not built here (oracle/Makefile builds it where the "
+                    "reference sources are present)")
+    if not shutil.which("perl"):
+        pytest.skip("perl is not installed")
     base = tmp_path_factory.mktemp("acceptance")
     return base, _install(str(base / "bin_ref"), "ref"), _install(str(base / "bin_ours"), "ours")
 

@@ -7,7 +7,9 @@ shows with many tiles, long runs or the exit test):
   C2  configs[1] at 1/5 scale (SURVEY.md section 6's probe): 2 M single-end reads with qualities x 50 k transcripts, 20 rounds;
   C3  configs[2] subsample: 1 M paired-end reads with qualities (2 x 100) against the full 200 k transcripts, 20 rounds.
 
-Tolerance: north_star's 1e-6 relative on theta (>= 1e-7) and on the result rows' TPM (printed %.2f).
+Tolerance: 1e-6 relative on theta (>= 1e-7) and on the result rows' TPM (printed %.2f).  The reference's outputs are
+stored in tests/golden/ref_outputs.json.gz (tools/make_golden_ref.py); at these sizes theta, the model and the result
+rows are compared at a fixed seeded sample of ref_golden.KEEP positions each.
 """
 import os
 import re
@@ -15,6 +17,7 @@ import re
 import numpy as np
 import pytest
 
+import ref_golden
 import rsem_files as rf
 
 pytestmark = pytest.mark.gpu
@@ -23,8 +26,6 @@ THREADS = min(32, os.cpu_count() or 1)
 
 @pytest.fixture(scope="module")
 def workdir(tmp_path_factory, built):
-    if not rf.have_ref():
-        pytest.skip("oracle/_ref binaries not available")
     return tmp_path_factory.mktemp("baseline_sizes")
 
 
@@ -32,24 +33,19 @@ def _rounds(p):
     return [int(m.group(1)) for m in re.finditer(r"^ROUND = (\d+),", p.stdout, re.M)]
 
 
-def _compare_outputs(ref, ours, check_model=True):
-    raw_r, pol_r = rf.read_theta(f"{ref}/s.stat/s.theta")
-    raw_o, pol_o = rf.read_theta(f"{ours}/s.stat/s.theta")
+def _compare_outputs(g, ours):
+    """our outputs in directory ours against the stored reference run g"""
+    o = ref_golden.em_outputs(ours, ofg=False)
+    raw_o, raw_r = g.take(o, "theta_raw"), g["theta_raw"]
+    pol_o, pol_r = g.take(o, "theta_pol"), g["theta_pol"]
     assert rf.close_rel(raw_o, raw_r, 1e-6), rf.max_rel(raw_o, raw_r)
     assert rf.close_rel(pol_o, pol_r, 1e-6), rf.max_rel(pol_o, pol_r)
-    if check_model:
-        mr, mo = rf.read_tokens(f"{ref}/s.stat/s.model"), rf.read_tokens(f"{ours}/s.stat/s.model")
-        assert mr.shape == mo.shape and np.all(np.abs(mo - mr) <= 1e-9 + 1e-6 * np.abs(mr))
+    mo, mr = g.take(o, "model"), g["model"]
+    assert np.all(np.abs(mo - mr) <= 1e-9 + 1e-6 * np.abs(mr))
     for res in ("iso_res", "gene_res"):
-        a, b = rf.read_res(f"{ours}/s.temp/s.{res}"), rf.read_res(f"{ref}/s.temp/s.{res}")
-        assert len(a) == len(b)
-        for ra, rb in zip(a, b):
-            try:
-                xa, xb = np.array(ra, float), np.array(rb, float)
-            except ValueError:
-                assert ra == rb
-                continue
-            assert np.all(np.abs(xa - xb) <= 0.011 + 1e-6 * np.abs(xb))
+        assert g.same(o, res + "_layout")
+        xa, xb = g.take(o, res), g[res]
+        assert np.all(np.abs(xa - xb) <= 0.011 + 1e-6 * np.abs(xb))
     return rf.max_rel(raw_o, raw_r)
 
 
@@ -59,39 +55,37 @@ def c1_base(workdir):
 
 
 def test_c1_full_size_20_rounds(workdir, c1_base):
-    ref, ours = rf.clone(c1_base, str(workdir / "c1_20_ref")), rf.clone(c1_base, str(workdir / "c1_20_ours"))
-    pr = rf.run_em(ref, 0, "ref", rounds=20, threads=THREADS, gibbs_out=False)
+    ours = rf.clone(c1_base, str(workdir / "c1_20_ours"))
     po = rf.run_em(ours, 0, "ours", rounds=20, gibbs_out=False)
-    assert _rounds(pr) == _rounds(po) == list(range(1, 21))
-    _compare_outputs(ref, ours)
+    g = ref_golden.Run("baseline/c1_20")
+    assert list(g["rounds"]) == _rounds(po) == list(range(1, 21))
+    _compare_outputs(g, ours)
 
 
 def test_c1_free_running_to_convergence(workdir, c1_base):
     """no round override on either side: MIN_ROUND 20, MAX_ROUND 10000, stop when no theta >= 1e-7 moves by >= 1e-3
     (EM.cpp:406-416); the stop test runs on the device in chunks of 32 rounds and must end on the reference's round"""
-    ref, ours = rf.clone(c1_base, str(workdir / "c1_free_ref")), rf.clone(c1_base, str(workdir / "c1_free_ours"))
-    pr = rf.run_em(ref, 0, "ref_unpatched", threads=THREADS, gibbs_out=False)
+    ours = rf.clone(c1_base, str(workdir / "c1_free_ours"))
     po = rf.run_em(ours, 0, "ours", gibbs_out=False)
-    rr, ro = _rounds(pr), _rounds(po)
-    assert len(rr) > 20, "the data set is expected to need more than MIN_ROUND rounds"
-    assert ro[-1] == rr[-1], f"exit round differs: ours {ro[-1]}, reference {rr[-1]}"
-    assert ("Warning: RSEM reaches" in pr.stderr) == ("Warning: RSEM reaches" in po.stderr)
-    _compare_outputs(ref, ours)
+    g = ref_golden.Run("baseline/c1_free")     # the unpatched reference binary with -p 32
+    exit_ref, ro = int(g["exit_round"][0]), _rounds(po)
+    assert ro == list(range(1, len(ro) + 1)) and len(ro) > 20, "the data set is expected to need more than MIN_ROUND rounds"
+    assert ro[-1] == exit_ref, f"exit round differs: ours {ro[-1]}, reference {exit_ref}"
+    assert bool(g["max_round_warning"][0]) == ("Warning: RSEM reaches" in po.stderr)
+    _compare_outputs(g, ours)
 
 
 def test_c2_fifth_scale_20_rounds(workdir):
     base = rf.gen_dataset(str(workdir / "c2_base"), read_type=1, M=50_000, N1=2_000_000, N0=100_000, avg_family=10, read_len=100, seed=11)
-    ref, ours = rf.clone(base, str(workdir / "c2_ref")), rf.clone(base, str(workdir / "c2_ours"))
-    pr = rf.run_em(ref, 1, "ref", rounds=20, threads=os.cpu_count() or 1, gibbs_out=False)
-    po = rf.run_em(ours, 1, "ours", rounds=20, threads=THREADS, gibbs_out=False)
-    assert _rounds(pr) == _rounds(po) == list(range(1, 21))
-    _compare_outputs(ref, ours)
+    po = rf.run_em(base, 1, "ours", rounds=20, threads=THREADS, gibbs_out=False)
+    g = ref_golden.Run("baseline/c2")
+    assert list(g["rounds"]) == _rounds(po) == list(range(1, 21))
+    _compare_outputs(g, base)
 
 
 def test_c3_subsample_20_rounds(workdir):
     base = rf.gen_dataset(str(workdir / "c3_base"), read_type=3, M=200_000, N1=1_000_000, N0=50_000, avg_family=20, read_len=100, seed=11)
-    ref, ours = rf.clone(base, str(workdir / "c3_ref")), rf.clone(base, str(workdir / "c3_ours"))
-    pr = rf.run_em(ref, 3, "ref", rounds=20, threads=os.cpu_count() or 1, gibbs_out=False)
-    po = rf.run_em(ours, 3, "ours", rounds=20, threads=THREADS, gibbs_out=False)
-    assert _rounds(pr) == _rounds(po) == list(range(1, 21))
-    _compare_outputs(ref, ours)
+    po = rf.run_em(base, 3, "ours", rounds=20, threads=THREADS, gibbs_out=False)
+    g = ref_golden.Run("baseline/c3")
+    assert list(g["rounds"]) == _rounds(po) == list(range(1, 21))
+    _compare_outputs(g, base)

@@ -2,7 +2,6 @@
 E-step + allreduce + M-step flow over torch.distributed (gloo, world_size 2) against the single-process oracle.
 The oracle stands in for the CUDA kernel here (tests only); the collective and the sharding are the real code."""
 import os
-import re
 
 import numpy as np
 import pytest
@@ -10,6 +9,7 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
+import ref_golden
 import rsem_files as rf
 import synth
 import rsem_b200
@@ -28,11 +28,11 @@ def slice_csr(row_ptr, first, last):
 
 @pytest.mark.parametrize("threads", [2, 3, 7])
 def test_shards_equal_reference_thread_split(tmp_path, built, threads):
-    if not rf.have_ref():
-        pytest.skip("oracle/_ref binaries not available")
+    """the reference's rsem-run-em -p threads prints its split ("Thread t : N = .., NHit = .."): stored in
+    tests/golden/ref_outputs.json.gz (tools/make_golden_ref.py)"""
     d = rf.gen_dataset(str(tmp_path / "d"), read_type=0, M=80, N1=900, N0=40, read_len=40, maxL=100, seed=threads)
-    p = rf.run_em(d, 0, "ref", rounds=1, min_rounds=1, threads=threads, gibbs_out=False)
-    ref = [(int(a), int(b)) for a, b in re.findall(r"Thread \d+ : N = (\d+), NHit = (\d+)", p.stdout)]
+    ref = [(int(a), int(b)) for a, b in ref_golden.Run(f"sharding/{threads}")["split"].reshape(-1, 2)]
+    assert len(ref) == threads
     row_ptr, _, _, _ = rf.read_dat(f"{d}/s.temp/s.dat", False)
     mine = [(b - a, int(row_ptr[b] - row_ptr[a])) for a, b in shard_reads(row_ptr, threads)]
     assert mine == ref
